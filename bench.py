@@ -9,6 +9,8 @@ A "step" is one full pass of the hot path over one batch: 4 prompts per GPU x 10
 guidance (effective batch 8; API defaults guidance 5 / rescale 0.75 / eta 1, api/ezaudio.py:102) + VAE decode (BASELINE configs C2/C3).
 `value` times the loop with inputs resident in HBM; `e2e` times the public API call (`EzAudio.generate_audio`) with
 host-resident cached T5 embeddings (pinned) copied in and the waveforms copied back out every step.
+`--dump-outputs DIR` writes the waveforms of the last timed step of that loop (rank 0) to DIR/waveform.npy, float32 [prompts, 1, samples];
+weights, prompts and noise are seeded, so two builds run with the same arguments can be compared output for output.
 
 The same line also carries (N = 1; cheap legs, a few seconds each):
   parity   measured max / mean-abs of the BENCHMARKED precision on the reference's own golden output (tests/golden/dit_XL.npz, written by the
@@ -205,7 +207,10 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-cfg", action="store_true")
     ap.add_argument("--no-extras", action="store_true", help="skip the parity / bf16x3 / C4 / C5 legs")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="--impl ours: write the waveforms of the last timed step to DIR/waveform.npy")
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
     # stdout carries exactly ONE JSON line: library banners (e.g. "NCCL version ...") are sent to stderr
     sys.stdout.flush()
     real_stdout = os.dup(1)
@@ -294,6 +299,10 @@ def main():
     clk = clocks.stop()
     launches = int(Lb.ezb_launch_count() - n0)
     assert torch.isfinite(wav).all()
+    if a.dump_outputs and rank == 0:
+        import numpy as np
+        os.makedirs(a.dump_outputs, exist_ok=True)
+        np.save(os.path.join(a.dump_outputs, "waveform.npy"), wav.float().cpu().numpy())
     # ---- end to end through the public API (host buffers in / out)
     step_e2e()
     sync_all()

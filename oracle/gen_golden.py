@@ -1,6 +1,12 @@
-"""Generates tests/golden/*.npz by running the UNMODIFIED reference modules (imported from
-/root/reference, CPU fp32) on the deterministic synthetic checkpoint + inputs.
+"""Generates tests/golden/*.npz by running the UNMODIFIED reference modules (CPU fp32, imported from the
+tree oracle/refimport.py finds) on the deterministic synthetic checkpoint + inputs, and tests/golden/weight_shapes.json.gz
+from the reference modules' state dicts.
 Run in the build container:  python oracle/gen_golden.py     -- TEST INFRASTRUCTURE."""
+import contextlib
+import copy
+import gzip
+import io
+import json
 import os
 import sys
 
@@ -20,7 +26,7 @@ def checksum(sd):
 
 
 @torch.no_grad()
-def dit_case(ref, name, cfg, B, L, Lc, seed, inpaint, tscalar=None, tvec=None):
+def dit_case(ref, name, cfg, B, L, Lc, seed, inpaint, tscalar=None, tvec=None, out_stride=1):
     sd = weights.synthetic_state_dict(weights.dit_param_shapes(cfg), seed)
     m = refimport.build(ref.MaskDiT, sd, **cfg)
     x = synth.synth_latents(B, L)
@@ -31,9 +37,10 @@ def dit_case(ref, name, cfg, B, L, Lc, seed, inpaint, tscalar=None, tvec=None):
     t = torch.tensor(tscalar) if tvec is None else torch.tensor(tvec, dtype=torch.long)
     gt, gm = (synth.synth_gt(B, L) if inpaint else (None, None))
     out, mae = m(x, t, ctx, context_mask=mask, gt=None if gt is None else gt.clone(), mae_mask_infer=gm)
-    np.savez_compressed(os.path.join(OUT, name + ".npz"), out=out.numpy(), sd_checksum=checksum(sd),
+    # config-scale cases keep every `out_stride`-th token (a full 30-s XL output is 1.5 MB)
+    np.savez_compressed(os.path.join(OUT, name + ".npz"), out=out[..., ::out_stride].numpy(), sd_checksum=checksum(sd),
                         x_checksum=float(x.double().abs().sum()), seed=seed, B=B, L=L, Lc=Lc,
-                        inpaint=inpaint, t=t.numpy())
+                        inpaint=inpaint, t=t.numpy(), **({"out_stride": out_stride} if out_stride > 1 else {}))
     print(name, tuple(out.shape), float(out.std()), float(out.abs().max()))
 
 
@@ -59,12 +66,15 @@ def controlnet_case(ref, name, cfg, B, L, Lc, seed, skip_stride=1):
 
 
 @torch.no_grad()
-def vae_case(ref, name, dcfg, B, L, seed):
+def vae_case(ref, name, dcfg, B, L, seed, out_stride=1):
     sd = weights.synthetic_state_dict(weights.vae_decoder_param_shapes(dcfg), seed)
     m = refimport.build(ref.OobleckDecoder, {k[len("decoder."):]: v for k, v in sd.items()}, **dcfg)
     z = synth.synth_latents(B, L, dcfg["latent_dim"], seed=31)
     wav = m(z)
-    np.savez_compressed(os.path.join(OUT, name + ".npz"), out=wav.numpy(), sd_checksum=checksum(sd), seed=seed, B=B, L=L)
+    # config-scale cases keep every `out_stride`-th sample (a full 10-s stereo batch is 1.9 MB); a stride prime to the 480-sample
+    # latent hop still visits every phase of the upsampling chain
+    np.savez_compressed(os.path.join(OUT, name + ".npz"), out=wav[..., ::out_stride].numpy(), sd_checksum=checksum(sd), seed=seed, B=B, L=L,
+                        **({"out_stride": out_stride} if out_stride > 1 else {}))
     print(name, tuple(wav.shape), float(wav.std()), float(wav.abs().max()))
 
 
@@ -105,19 +115,33 @@ def t5_case(ref, name, cfg, B, L, seed):
     print(name, tuple(out.shape), float(out.std()), float(out.abs().max()))
 
 
+def weight_shapes(ref, name):
+    """State-dict key -> shape of the reference MaskDiT (XL, L) and DiTControlNet (L), built on the meta device."""
+    shapes = {}
+    for key, cls, kw in (("MaskDiT_xl", ref.MaskDiT, synth.model_cfg("xl")), ("MaskDiT_l", ref.MaskDiT, synth.model_cfg("l")),
+                         ("DiTControlNet_l", ref.DiTControlNet, dict(synth.model_cfg("l"), **synth.CONTROLNET))):
+        with torch.device("meta"), contextlib.redirect_stdout(io.StringIO()):
+            m = cls(**copy.deepcopy(kw))
+        shapes[key] = {k: list(v.shape) for k, v in m.state_dict().items()}
+    with open(os.path.join(OUT, name + ".json.gz"), "wb") as f:
+        f.write(gzip.compress(json.dumps(shapes).encode(), mtime=0))
+    print(name, {k: len(v) for k, v in shapes.items()})
+
+
 def main():
     ref = refimport.import_reference()
     assert ref is not None, "reference tree not found"
     os.makedirs(OUT, exist_ok=True)
     torch.set_num_threads(os.cpu_count())
     only = set(sys.argv[1:])
-    global dit_case, controlnet_case, vae_case, vae_enc_case, energy_case, t5_case
+    global dit_case, controlnet_case, vae_case, vae_enc_case, energy_case, t5_case, weight_shapes
     if only:
         def filt(f):
             return lambda ref, name, *a, **k: f(ref, name, *a, **k) if name in only else None
         dit_case, controlnet_case, vae_case, vae_enc_case = filt(dit_case), filt(controlnet_case), filt(vae_case), filt(vae_enc_case)
         energy_case = filt(energy_case)
         t5_case = filt(t5_case)
+        weight_shapes = filt(weight_shapes)
     dit_case(ref, "dit_tiny72", synth.tiny_model(72), B=2, L=40, Lc=12, seed=3, inpaint=False, tscalar=999)
     dit_case(ref, "dit_tiny72_inpaint", synth.tiny_model(72), B=3, L=52, Lc=12, seed=3, inpaint=True, tvec=[999, 500, 19])
     dit_case(ref, "dit_tiny64", synth.tiny_model(64, heads=4, depth=2), B=2, L=130, Lc=100, seed=4, inpaint=False, tscalar=259)
@@ -135,10 +159,11 @@ def main():
     dit_case(ref, "dit_L_c1", synth.model_cfg("l"), B=1, L=256, Lc=100, seed=1, inpaint=False, tscalar=999)  # BASELINE config 1
     dit_case(ref, "dit_XL", synth.model_cfg("xl"), B=2, L=500, Lc=100, seed=2, inpaint=False, tscalar=479)
     # ---- configuration-scale cases (BASELINE configs C4 / C5 and the 10-s codec the benchmark times)
-    controlnet_case(ref, "controlnet_XL", synth.model_cfg("xl"), B=2, L=500, Lc=100, seed=2, skip_stride=10)      # C4 shapes (B_eff = 2)
-    dit_case(ref, "dit_XL_inpaint_30s", synth.model_cfg("xl"), B=2, L=1500, Lc=100, seed=2, inpaint=True, tvec=[989, 9])  # C5 shapes
-    vae_case(ref, "vae_full_10s", synth.VAE_DECODER, B=2, L=500, seed=6)
+    controlnet_case(ref, "controlnet_XL", synth.model_cfg("xl"), B=2, L=500, Lc=100, seed=2, skip_stride=20)      # C4 shapes (B_eff = 2)
+    dit_case(ref, "dit_XL_inpaint_30s", synth.model_cfg("xl"), B=2, L=1500, Lc=100, seed=2, inpaint=True, tvec=[989, 9], out_stride=2)  # C5 shapes
+    vae_case(ref, "vae_full_10s", synth.VAE_DECODER, B=2, L=500, seed=6, out_stride=7)
     vae_enc_case(ref, "vae_enc_full_10s", synth.VAE_ENCODER, B=1, T=480 * 500, seed=8)
+    weight_shapes(ref, "weight_shapes")
 
 
 if __name__ == "__main__":

@@ -27,6 +27,11 @@ def load_golden(name):
     return np.load(os.path.join(GOLDEN, name + ".npz"))
 
 
+def sampled(x, g):
+    """The entries of a full output `x` that golden `g` stores: config-scale goldens keep every `out_stride`-th entry of the last axis."""
+    return x[..., ::int(g["out_stride"])] if "out_stride" in g.files else x
+
+
 def dit_case_inputs(name):
     """-> cfg, sd, dict(x, t, ctx, mask, gt, gt_mask), golden npz."""
     mk, kw = DIT_CASES[name]

@@ -65,23 +65,17 @@ def test_scheduler_matches_oracle_restatement_and_invariants():
                 assert torch.allclose(mine, o.step(v, t, x, eta, z), atol=2e-6)
 
 
-def test_weight_wire_format_matches_live_reference():
-    from oracle import refimport
-    ref = refimport.import_reference()
-    if ref is None:
-        pytest.skip("reference tree not present")
-    import contextlib
-    import copy
-    import io
+def test_weight_wire_format_matches_reference_golden():
+    """State-dict keys / shapes the loader expects == those of the unmodified reference MaskDiT (XL, L) and DiTControlNet (L)
+    (tests/golden/weight_shapes.json.gz, written by oracle/gen_golden.py)."""
+    import gzip
+    import json
     from ezaudio_b200 import synth, weights
-    for cfg in (synth.model_cfg("xl"), synth.model_cfg("l")):
-        with torch.device("meta"), contextlib.redirect_stdout(io.StringIO()):
-            m = ref.MaskDiT(**copy.deepcopy(cfg))
-        assert {k: tuple(v.shape) for k, v in m.state_dict().items()} == dict(weights.dit_param_shapes(cfg))
-    cfg = synth.model_cfg("l")
-    with torch.device("meta"), contextlib.redirect_stdout(io.StringIO()):
-        c = ref.DiTControlNet(**copy.deepcopy(cfg), **copy.deepcopy(synth.CONTROLNET))
-    assert {k: tuple(v.shape) for k, v in c.state_dict().items()} == dict(weights.controlnet_param_shapes(cfg, synth.CONTROLNET))
+    with gzip.open(os.path.join(ROOT, "tests", "golden", "weight_shapes.json.gz"), "rt") as f:
+        want = {model: {k: tuple(v) for k, v in shapes.items()} for model, shapes in json.load(f).items()}
+    assert want["MaskDiT_xl"] == dict(weights.dit_param_shapes(synth.model_cfg("xl")))
+    assert want["MaskDiT_l"] == dict(weights.dit_param_shapes(synth.model_cfg("l")))
+    assert want["DiTControlNet_l"] == dict(weights.controlnet_param_shapes(synth.model_cfg("l"), synth.CONTROLNET))
 
 
 def test_shard_range_covers_everything_once():

@@ -19,7 +19,7 @@ def test_dit_oracle_matches_reference_golden(name):
     cfg, sd, inp, g = helpers.dit_case_inputs(name)
     with torch.no_grad():
         out, _ = O.maskdit_forward(sd, cfg, inp["x"], inp["t"], inp["ctx"], inp["mask"], inp["gt"], inp["gt_mask"])
-    err = float((out - torch.from_numpy(g["out"])).abs().max())
+    err = float((helpers.sampled(out, g) - torch.from_numpy(g["out"])).abs().max())
     assert err < TOL, err
 
 
@@ -53,7 +53,9 @@ def test_vae_oracle_matches_reference_golden(name, dcfg, B, L):
     with torch.no_grad():
         wav = O.vae_decode(sd, z, strides=tuple(dcfg["strides"]))
     ref = torch.from_numpy(g["out"])
-    assert wav.shape == ref.shape == (B, 1, 480 * L)
+    assert wav.shape == (B, 1, 480 * L)
+    wav = helpers.sampled(wav, g)
+    assert wav.shape == ref.shape
     assert float((wav - ref).abs().max()) < 1e-5 + 1e-4 * float(ref.abs().max())
 
 
